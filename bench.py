@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- gradient-steps/sec of the OSRL per-step hot path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload = BASELINE.json configs[1]: BCQ-Lag, OfflineCarCircle-v0-shaped transitions (obs 8, act 2),
 batch 256 per GPU, hidden [256,256] x2, VAE 400, 10 sampled actions, 2+2 double-Q nets, fp32.
@@ -25,6 +25,11 @@ Extra keys of the result line: `roofline` -- step-level fraction of the measured
 `roofline.kernels`; `other_configs` -- short device-resident runs of BASELINE.json configs[2..4] (CPQ B=512,
 CDT B=2048 seq 10, BEAR-Lag B=512 per GPU and the strong-scaling BEAR-Lag global B=4096) with ms/step and the same
 step-level fractions; `cpu_baseline`.
+
+--dump-outputs DIR (ours, rank 0): after the K timed steps, what the last of them left for a caller -- the step's
+statistics (float32), the PID / dual scalars (float64) and every trained and target parameter tensor (float32, 6.3 MB)
+-- as DIR/<name>.npy.  Model init, dataset and device sampling are seeded, so the same arguments give the same inputs
+and two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -280,6 +285,17 @@ def run_preprocess(local: int, rows: int = 1_000_000, ep_len: int = 1000):
             "first_returns_equal_oracle": ok, "episodes": int(eng.n_traj)}
 
 
+def dump_outputs(out_dir: str, eng) -> None:
+    """The engine's outputs after its last step (statistics, scalars, parameters) as out_dir/<name>.npy; '/' in a
+    name becomes '.'."""
+    arrays = {f"stats.{k}": np.float32(v) for k, v in eng.stats().items()}
+    arrays.update({f"scalars.{k}": np.float64(v) for k, v in eng.scalars().items()})
+    arrays.update({f"params.{k}": v.numpy() for k, v in eng.read_params().items()})
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name.replace("/", ".") + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------ reference arm
 def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
@@ -384,6 +400,8 @@ def run_ours(args):
     ms = e0.elapsed_time(e1)
     launches = eng.launches - l0
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, eng)
     if world > 1:
         t = torch.tensor([ms], device="cuda")
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -625,6 +643,8 @@ def main():
     ap.add_argument("--steps", type=int, default=2000)
     ap.add_argument("--warmup", type=int, default=50)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

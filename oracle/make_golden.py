@@ -106,50 +106,112 @@ def rel_err(a: torch.Tensor, b: torch.Tensor) -> float:
     return float((a - b).abs().max()) / den
 
 
-def run_case(osrl, name, algo, cfg, B, steps, full):
-    init_seed, data_seed, noise_seed = 0, 1234, 4321
+# ---- reference results kept small: tests/test_cpu_oracle_hparams.py holds the oracle to what the reference computed at
+# configurations away from the fixtures; it stores each final tensor's max |x|, checksum and a fixed sample of entries
+PIN_SAMPLE = 8
+
+
+def pin_tensor(t: torch.Tensor) -> dict:
+    a = t.detach().double().reshape(-1).numpy()
+    idx = np.sort(np.random.default_rng(0).choice(a.size, min(PIN_SAMPLE, a.size), replace=False)).astype(np.int32)
+    return {"max": float(np.abs(a).max()), "checksum": checksum(t), "idx": idx, "val": a[idx].astype(np.float32)}
+
+
+def pin_run(run: dict) -> dict:
+    """What check_run needs of a reference run: initial parameters as digests, final parameters pinned, the rest (stats,
+    scalars) as is."""
+    from tests.helpers import digest
+    return dict(run, init={k: digest(v) for k, v in run["init"].items()},
+                stats=[{k: float(v) for k, v in r.items()} for r in run["stats"]],
+                final={k: pin_tensor(v) for k, v in run["final"].items()})
+
+
+def _param_err(got: torch.Tensor, want) -> float:
+    """max |got - want| / max |want| for a full tensor; for a pinned one, the largest ratio among the bounds that
+    max |got - want| <= tol max |want| implies (max |x|, the sampled entries, the checksums)."""
+    if isinstance(want, torch.Tensor):
+        return rel_err(got, want)
+    a = got.detach().double().reshape(-1)
+    m, n = want["max"], a.numel()
+    den = m + 1e-30
+    sampled = a[torch.tensor(want["idx"], dtype=torch.long)] - torch.tensor(want["val"], dtype=torch.float64)
+    errs = [abs(float(a.abs().max()) - m) / den, float(sampled.abs().max()) / den]
+    got_sum = checksum(got)
+    for i, (g, w) in enumerate(zip(got_sum, want["checksum"])):
+        scale = n * den * ((2 * m + 1e-30) if i == 2 else 1.0)   # sum(a^2 - b^2) <= sum |a - b| |a + b|
+        errs.append(abs(g - w) / scale)
+    return max(errs)
+
+
+def check_run(name, want, got, stat_tol, stat_den, param_tol, skip_params=()):
+    """got (an oracle run) against want (a reference run, full or pinned): same initial parameters bit for bit,
+    per-step stats within stat_tol relative, final parameters within param_tol of each tensor's max |x|."""
+    from tests.helpers import digest
+    assert list(want["init"]) == list(got["init"]), (name, "state_dict keys differ")
+    for k, v in want["init"].items():
+        same = torch.equal(v, got["init"][k]) if isinstance(v, torch.Tensor) else v == digest(got["init"][k])
+        assert same, (name, "init differs", k)
+    worst = 0.0
+    assert len(want["stats"]) == len(got["stats"])
+    for s, (r, o) in enumerate(zip(want["stats"], got["stats"])):
+        assert set(r) == set(o), (name, s, set(r) ^ set(o))
+        for k in r:
+            e = abs(r[k] - o[k]) / (abs(r[k]) + stat_den)
+            worst = max(worst, e)
+            assert e < stat_tol, (name, s, k, r[k], o[k])
+    perr = 0.0
+    for k, v in want["final"].items():
+        if any(x in k for x in skip_params):
+            continue
+        perr = max(perr, _param_err(got["final"][k], v))
+    assert perr < param_tol, (name, "final params differ", perr)
+    return worst, perr
+
+
+def make_batches(cfg, B, steps, data_seed=1234):
+    rng = np.random.default_rng(data_seed)
+    return [synth.make_batch(rng, B, cfg.state_dim, cfg.action_dim) for _ in range(steps)]
+
+
+def reference_run(osrl, algo, cfg, B, steps, init_seed=0, noise_seed=4321):
+    """The unmodified reference: initial parameters, per-step logged stats, final parameters."""
     torch.manual_seed(init_seed)
     ref_model, ref_trainer = build_reference(osrl, algo, cfg)
-    torch.manual_seed(init_seed)
-    orc = ORACLES[algo](cfg)
-    ref_sd = ref_model.state_dict()
-    assert list(ref_sd.keys()) == list(orc.params.keys()), (name, "state_dict keys differ")
-    for k, v in ref_sd.items():
-        assert torch.equal(v, orc.params[k]), (name, "init differs", k)
-    init = {k: v.clone() for k, v in orc.params.items()}
-
-    rng = np.random.default_rng(data_seed)
-    batches = [synth.make_batch(rng, B, cfg.state_dim, cfg.action_dim) for _ in range(steps)]
-
+    init = {k: v.clone() for k, v in ref_model.state_dict().items()}
     torch.manual_seed(noise_seed)
-    ref_stats = []
-    for b in batches:
+    stats = []
+    for b in make_batches(cfg, B, steps):
         n0 = len(ref_trainer.logger.rows)
         ref_trainer.train_one_step(*batch_args(algo, b))
         row = {}
         for r in ref_trainer.logger.rows[n0:]:
             row.update(r)
-        ref_stats.append(row)
+        stats.append(row)
+    return {"init": init, "stats": stats, "final": ref_model.state_dict()}
 
+
+def oracle_run(algo, cfg, B, steps, init_seed=0, noise_seed=4321):
+    """The oracle on the same seeds, batches and noise stream as reference_run (plus the batches and the noise)."""
+    torch.manual_seed(init_seed)
+    orc = ORACLES[algo](cfg)
+    init = {k: v.clone() for k, v in orc.params.items()}
+    batches = make_batches(cfg, B, steps)
     torch.manual_seed(noise_seed)
-    orc_stats, noises = [], []
+    stats, noises = [], []
     for b in batches:
-        orc_stats.append(orc.step(*batch_args(algo, b)))
+        stats.append(orc.step(*batch_args(algo, b)))
         noises.append({k: v.clone() for k, v in orc.last_noise.items()})
+    return {"init": init, "stats": stats, "final": orc.params, "batches": batches, "noises": noises}
 
-    worst = 0.0
-    for s, (r, o) in enumerate(zip(ref_stats, orc_stats)):
-        assert set(r) == set(o), (name, s, set(r) ^ set(o))
-        for k in r:
-            e = abs(r[k] - o[k]) / (abs(r[k]) + 1e-12)
-            worst = max(worst, e)
-            assert e < 2e-6, (name, s, k, r[k], o[k])
-    perr = 0.0
-    for k, v in ref_model.state_dict().items():
-        perr = max(perr, rel_err(orc.params[k], v))
-    assert perr < 2e-6, (name, "final params differ", perr)
+
+def run_case(osrl, name, algo, cfg, B, steps, full):
+    init_seed, data_seed, noise_seed = 0, 1234, 4321
+    ref = reference_run(osrl, algo, cfg, B, steps, init_seed, noise_seed)
+    orc = oracle_run(algo, cfg, B, steps, init_seed, noise_seed)
+    worst, perr = check_run(name, ref, orc, 2e-6, 1e-12, 2e-6)
     print(f"[golden] {name}: oracle == reference over {steps} steps (stat rel err {worst:.2e}, param rel err {perr:.2e})")
 
+    init, ref_stats, batches, noises = orc["init"], ref["stats"], orc["batches"], orc["noises"]
     out = {"meta": json.dumps({"algo": algo, "cfg": dataclasses.asdict(cfg), "B": B, "steps": steps,
                                "init_seed": init_seed, "data_seed": data_seed, "noise_seed": noise_seed,
                                "full": full, "torch": torch.__version__, "keys": list(init.keys()),
@@ -158,7 +220,7 @@ def run_case(osrl, name, algo, cfg, B, steps, full):
     if full:
         for k, v in init.items():
             out["init/" + k] = v.numpy()
-        for k, v in ref_model.state_dict().items():
+        for k, v in ref["final"].items():
             out["final/" + k] = v.numpy()
         for s, (b, nz) in enumerate(zip(batches, noises)):
             for k, v in b.items():
@@ -167,7 +229,7 @@ def run_case(osrl, name, algo, cfg, B, steps, full):
                 out[f"noise{s}/{k}"] = v.numpy()
     else:
         out["init_checksum"] = np.array([checksum(v) for v in init.values()])
-        out["final_checksum"] = np.array([checksum(v) for v in ref_model.state_dict().values()])
+        out["final_checksum"] = np.array([checksum(v) for v in ref["final"].values()])
         out["noise_checksum"] = np.array([[checksum(v) for v in nz.values()] for nz in noises])
     np.savez_compressed(os.path.join(OUT, name + ".npz"), **out)
 
@@ -250,7 +312,9 @@ class DropReplay:
         assert not self.q, f"{len(self.q)} dropout tensors were not consumed by the reference"
 
 
-def run_cdt_case(osrl, name, cfg, B, steps, full):
+def reference_cdt_run(osrl, cfg, B, steps):
+    """The unmodified CDT / CDTTrainer on replayed dropout multipliers: initial parameters, stats, final parameters,
+    log-temperature."""
     from oracle import cdt as ocdt
     torch.manual_seed(0)
     ref = osrl.algorithms.CDT(state_dim=cfg.state_dim, action_dim=cfg.action_dim, max_action=cfg.max_action,
@@ -264,44 +328,61 @@ def run_cdt_case(osrl, name, cfg, B, steps, full):
                                          weight_decay=cfg.weight_decay, betas=cfg.betas, clip_grad=cfg.clip_grad,
                                          lr_warmup_steps=cfg.lr_warmup_steps, loss_cost_weight=cfg.loss_cost_weight,
                                          loss_state_weight=cfg.loss_state_weight, device="cpu")
+    init = {k: v.clone() for k, v in ref.state_dict().items() if "causal_mask" not in k}
     torch.manual_seed(0)
-    orc = ocdt.CDTOracle(cfg)
-    sd = {k: v for k, v in ref.state_dict().items() if "causal_mask" not in k}
-    assert list(sd.keys()) == list(orc.params.keys()), (list(sd.keys())[:12], list(orc.params.keys())[:12])
-    for k, v in sd.items():
-        assert torch.equal(v, orc.params[k]), ("init differs", k)
-    init = {k: v.clone() for k, v in orc.params.items()}
-    rng = np.random.default_rng(77)
-    batches = [make_seq_batch(rng, B, cfg.seq_len, cfg.state_dim, cfg.action_dim) for _ in range(steps)]
-    ref_stats, orc_stats, all_masks = [], [], []
+    masker = ocdt.CDTOracle(cfg)          # draws the multipliers (and leaves torch's generator where the oracle does)
     mgen = torch.Generator().manual_seed(4242)
     ref.train()
-    for b in batches:
-        masks = orc.draw_masks(B, generator=mgen)       # empty when every dropout is 0
-        all_masks.append(masks)
+    stats = []
+    for b in make_cdt_batches(cfg, B, steps):
         n0 = len(trainer.logger.rows)
-        with DropReplay(masks.values()):
+        with DropReplay(masker.draw_masks(B, generator=mgen).values()):
             trainer.train_one_step(*[torch.from_numpy(b[k]) for k in CDT_KEYS])
         row = {}
         for r in trainer.logger.rows[n0:]:
             row.update(r)
-        ref_stats.append(row)
-        orc_stats.append(orc.step(*[torch.from_numpy(b[k]) for k in CDT_KEYS], noise=masks))
-    worst = 0.0
-    for s, (r, o) in enumerate(zip(ref_stats, orc_stats)):
-        assert set(r) == set(o), set(r) ^ set(o)
-        for k in r:
-            e = abs(r[k] - o[k]) / (abs(r[k]) + 1e-9)
-            worst = max(worst, e)
-            assert e < 2e-5, (name, s, k, r[k], o[k])
+        stats.append(row)
+    return {"init": init, "stats": stats, "log_temperature": float(ref.log_temperature.detach()),
+            "final": {k: v for k, v in ref.state_dict().items() if "causal_mask" not in k}}
+
+
+def make_cdt_batches(cfg, B, steps):
+    rng = np.random.default_rng(77)
+    return [make_seq_batch(rng, B, cfg.seq_len, cfg.state_dim, cfg.action_dim) for _ in range(steps)]
+
+
+def oracle_cdt_run(cfg, B, steps):
+    """oracle/cdt.py on the batches and dropout multipliers of reference_cdt_run (plus the batches and multipliers)."""
+    from oracle import cdt as ocdt
+    torch.manual_seed(0)
+    orc = ocdt.CDTOracle(cfg)
+    init = {k: v.clone() for k, v in orc.params.items()}
+    batches = make_cdt_batches(cfg, B, steps)
+    mgen = torch.Generator().manual_seed(4242)
+    stats, all_masks = [], []
+    for b in batches:
+        masks = orc.draw_masks(B, generator=mgen)       # empty when every dropout is 0
+        all_masks.append(masks)
+        stats.append(orc.step(*[torch.from_numpy(b[k]) for k in CDT_KEYS], noise=masks))
+    return {"init": init, "stats": stats, "final": orc.params, "log_temperature": float(orc.log_temperature),
+            "batches": batches, "masks": all_masks}
+
+
+def check_cdt_run(name, want, got):
     # in_proj_bias: the key-bias slice has an exactly-zero true gradient (softmax shift invariance); what
     # Adam sees there is rounding noise, so its sign-like update is not reproducible even by the reference
-    perr = max(rel_err(orc.params[k], v) for k, v in ref.state_dict().items()
-               if "causal_mask" not in k and "in_proj_bias" not in k)
-    assert perr < 2e-5, perr
-    lt = abs(float(ref.log_temperature) - float(orc.log_temperature))
+    worst, perr = check_run(name, want, got, 2e-5, 1e-9, 2e-5, skip_params=("in_proj_bias",))
+    lt = abs(want["log_temperature"] - got["log_temperature"])
     assert lt < 1e-9, lt
+    return worst, perr
+
+
+def run_cdt_case(osrl, name, cfg, B, steps, full):
+    ref = reference_cdt_run(osrl, cfg, B, steps)
+    orc = oracle_cdt_run(cfg, B, steps)
+    worst, perr = check_cdt_run(name, ref, orc)
     print(f"[golden] {name}: oracle == reference over {steps} steps (stat rel err {worst:.2e}, param rel err {perr:.2e})")
+    init, ref_stats, batches, all_masks = orc["init"], ref["stats"], orc["batches"], orc["masks"]
     cfgd = dataclasses.asdict(cfg)
     cfgd["betas"] = list(cfgd["betas"])
     out = {"meta": json.dumps({"algo": "cdt", "cfg": cfgd, "B": B, "steps": steps, "full": full,
@@ -311,18 +392,17 @@ def run_cdt_case(osrl, name, cfg, B, steps, full):
     if full:
         for k, v in init.items():
             out["init/" + k] = v.numpy()
-        for k, v in ref.state_dict().items():
-            if "causal_mask" not in k:
-                out["final/" + k] = v.numpy()
+        for k, v in ref["final"].items():
+            out["final/" + k] = v.numpy()
         for s, b in enumerate(batches):
             for k, v in b.items():
                 out[f"batch{s}/{k}"] = v
             for k, v in all_masks[s].items():          # keep bits; the multiplier is bit / (1 - p)
                 out[f"drop{s}/{k}"] = np.packbits((v.numpy() > 0).reshape(-1))
-        out["log_temperature"] = np.array(float(ref.log_temperature))
+        out["log_temperature"] = np.array(ref["log_temperature"])
     else:
         out["init_checksum"] = np.array([checksum(v) for v in init.values()])
-        out["final_checksum"] = np.array([checksum(v) for k, v in ref.state_dict().items() if "causal_mask" not in k])
+        out["final_checksum"] = np.array([checksum(v) for v in ref["final"].values()])
     np.savez_compressed(os.path.join(OUT, name + ".npz"), **out)
 
 
@@ -395,67 +475,98 @@ def main_coptidice():
     run_coptidice_case(osrl, "coptidice_small", cfg, 32, 4)
 
 
-def run_coptidice_case(osrl, name, cfg, B, steps):
-    """oracle.coptidice == the unmodified reference over `steps` steps at configuration `cfg` (asserted), fixture
-    written to OUT/<name>.npz."""
-    from oracle import coptidice as oc
+COP_KEYS = ("observations", "next_observations", "actions", "rewards", "costs", "done")
+
+
+def coptidice_inputs(cfg, B, steps):
+    """observations_std, actions_std and the batches (with is_init) of a COptiDICE case, seeded"""
     rng = np.random.default_rng(21)
     obs_std = rng.uniform(0.5, 1.5, (1, cfg.state_dim)).astype(np.float32)
     act_std = rng.uniform(0.3, 0.8, (1, cfg.action_dim)).astype(np.float32)
+    batches = []
+    for _ in range(steps):
+        b = synth.make_batch(rng, B, cfg.state_dim, cfg.action_dim)
+        b["is_init"] = (rng.random(B) < 0.25).astype(np.float32)
+        batches.append(b)
+    return obs_std, act_std, batches
+
+
+def _cop_args(b):
+    return [torch.from_numpy(b[k]) for k in COP_KEYS] + [torch.from_numpy(b["is_init"])]
+
+
+def reference_coptidice_run(osrl, cfg, B, steps):
+    """The unmodified COptiDICE / COptiDICETrainer: initial parameters, stats, final parameters, tau and lambda."""
+    obs_std, act_std, batches = coptidice_inputs(cfg, B, steps)
     torch.manual_seed(0)
     ref = osrl.algorithms.COptiDICE(cfg.state_dim, cfg.action_dim, cfg.max_action, cfg.f_type, cfg.init_state_propotion,
                                     obs_std, act_std, cfg.a_hidden_sizes, cfg.c_hidden_sizes, cfg.gamma, cfg.alpha,
                                     cfg.cost_ub_epsilon, cfg.num_nu, cfg.num_chi, cfg.cost_limit, cfg.episode_len, "cpu")
     trainer = osrl.algorithms.COptiDICETrainer(ref, None, logger=ref_shim.NullLogger(), actor_lr=cfg.actor_lr,
                                                critic_lr=cfg.critic_lr, scalar_lr=cfg.scalar_lr, device="cpu")
-    torch.manual_seed(0)
-    orc = oc.COptiDICEOracle(cfg, obs_std, act_std)
-    sd = ref.state_dict()
-    assert list(sd.keys()) == [k for k in orc.params if k not in ("tau", "lmbda")], list(sd.keys())[:8]
-    for k, v in sd.items():
-        assert torch.equal(v, orc.params[k]), ("init differs", k)
-    init = {k: v.clone() for k, v in orc.params.items()}
-    keys = ("observations", "next_observations", "actions", "rewards", "costs", "done")
-    out = {}
-    worst = 0.0
-    stats_all = []
-    for s in range(steps):
-        b = synth.make_batch(rng, B, cfg.state_dim, cfg.action_dim)
-        b["is_init"] = (rng.random(B) < 0.25).astype(np.float32)
-        args = [torch.from_numpy(b[k]) for k in keys] + [torch.from_numpy(b["is_init"])]
+    scalars = {"tau": ref.tau, "lmbda": ref.lmbda}           # (parameters outside the state_dict)
+    init = {k: v.detach().clone() for k, v in {**ref.state_dict(), **scalars}.items()}
+    stats = []
+    for s, b in enumerate(batches):
         n0 = len(trainer.logger.rows)
         torch.manual_seed(1000 + s)
-        trainer.train_one_step(args)
+        trainer.train_one_step(_cop_args(b))
         row = {}
         for r in trainer.logger.rows[n0:]:
             row.update(r)
+        stats.append(row)
+    return {"init": init, "stats": stats, "final": {k: v.detach() for k, v in {**ref.state_dict(), **scalars}.items()},
+            "tau": float(ref.tau.detach()), "lmbda": float(ref.lmbda.detach())}
+
+
+def oracle_coptidice_run(cfg, B, steps):
+    """oracle/coptidice.py on the inputs of reference_coptidice_run (plus the inputs and the noise)."""
+    from oracle import coptidice as oc
+    obs_std, act_std, batches = coptidice_inputs(cfg, B, steps)
+    torch.manual_seed(0)
+    orc = oc.COptiDICEOracle(cfg, obs_std, act_std)
+    init = {k: v.clone() for k, v in orc.params.items()}
+    stats, noises = [], []
+    for s, b in enumerate(batches):
         torch.manual_seed(1000 + s)
-        got = orc.step(*args)
-        assert set(row) == set(got), set(row) ^ set(got)
-        for k in row:
-            e = abs(row[k] - got[k]) / (abs(row[k]) + 1e-6)
-            worst = max(worst, e)
-            assert e < 2e-5, (s, k, row[k], got[k])
-        stats_all.append([row[k] for k in sorted(row)])
-        for k, v in b.items():
-            out[f"batch{s}/{k}"] = v
-        for k, v in orc.last_noise.items():
-            out[f"noise{s}/{k}"] = v.numpy()
-    perr = max(rel_err(orc.params[k], v) for k, v in ref.state_dict().items())
-    serr = max(abs(float(ref.tau) - float(orc.params["tau"])), abs(float(ref.lmbda) - float(orc.params["lmbda"])))
-    assert perr < 2e-5 and serr < 1e-6, (perr, serr)
+        stats.append(orc.step(*_cop_args(b)))
+        noises.append({k: v.clone() for k, v in orc.last_noise.items()})
+    return {"init": init, "stats": stats, "final": orc.params, "tau": float(orc.params["tau"]),
+            "lmbda": float(orc.params["lmbda"]), "obs_std": obs_std, "act_std": act_std, "batches": batches,
+            "noises": noises}
+
+
+def check_coptidice_run(name, want, got):
+    worst, perr = check_run(name, want, got, 2e-5, 1e-6, 2e-5)
+    serr = max(abs(want["tau"] - got["tau"]), abs(want["lmbda"] - got["lmbda"]))
+    assert serr < 1e-6, serr
+    return worst, perr, serr
+
+
+def run_coptidice_case(osrl, name, cfg, B, steps):
+    """oracle.coptidice == the unmodified reference over `steps` steps at configuration `cfg` (asserted), fixture
+    written to OUT/<name>.npz."""
+    ref = reference_coptidice_run(osrl, cfg, B, steps)
+    orc = oracle_coptidice_run(cfg, B, steps)
+    worst, perr, serr = check_coptidice_run(name, ref, orc)
     print(f"[golden] {name}: oracle == reference over {steps} steps (stat rel err {worst:.2e}, "
           f"param rel err {perr:.2e}, tau/lambda abs err {serr:.1e})")
+    out = {}
+    for s, (b, nz) in enumerate(zip(orc["batches"], orc["noises"])):
+        for k, v in b.items():
+            out[f"batch{s}/{k}"] = v
+        for k, v in nz.items():
+            out[f"noise{s}/{k}"] = v.numpy()
     cfgd = dataclasses.asdict(cfg)
-    out["meta"] = json.dumps({"algo": "coptidice", "cfg": cfgd, "B": B, "steps": steps, "keys": list(init.keys()),
-                              "stat_keys": sorted(row.keys()), "torch": torch.__version__})
-    out["stats"] = np.array(stats_all, dtype=np.float64)
-    out["observations_std"], out["actions_std"] = obs_std, act_std
-    for k, v in init.items():
+    out["meta"] = json.dumps({"algo": "coptidice", "cfg": cfgd, "B": B, "steps": steps,
+                              "keys": list(orc["init"].keys()),
+                              "stat_keys": sorted(ref["stats"][0].keys()), "torch": torch.__version__})
+    out["stats"] = np.array([[r[k] for k in sorted(r)] for r in ref["stats"]], dtype=np.float64)
+    out["observations_std"], out["actions_std"] = orc["obs_std"], orc["act_std"]
+    for k, v in orc["init"].items():
         out["init/" + k] = v.numpy()
-    for k, v in ref.state_dict().items():
+    for k, v in ref["final"].items():
         out["final/" + k] = v.numpy()
-    out["final/tau"], out["final/lmbda"] = ref.tau.detach().numpy(), ref.lmbda.detach().numpy()
     np.savez_compressed(os.path.join(OUT, name + ".npz"), **out)
 
 

@@ -1,5 +1,6 @@
 """Shared helpers of the parity tests (the oracle is the checker, never the product)."""
 import copy
+import hashlib
 import json
 import os
 
@@ -19,6 +20,64 @@ def load_golden(name):
     z = np.load(os.path.join(GOLDEN, name + ".npz"), allow_pickle=False)
     meta = json.loads(str(z["meta"]))
     return z, meta
+
+
+# ---- what the unmodified reference computed, stored so that the comparisons with it run anywhere.  A pin is a nested
+# structure of dicts (str keys), lists, tuples, scalars and numpy arrays; oracle/record_reference.py writes one per test
+# module as tests/golden/reference_<name>.npz: the structure as JSON, the arrays' bytes back to back in one member.
+def save_pin(name, obj):
+    blob = []
+    size = 0
+
+    def enc(x):
+        nonlocal size
+        if isinstance(x, np.ndarray):
+            blob.append(x.tobytes())      # (C order)
+            size += x.nbytes
+            return {"__array__": [x.dtype.str, list(x.shape), size - x.nbytes]}
+        if isinstance(x, dict):
+            assert all(isinstance(k, str) and not k.startswith("__") for k in x), list(x)
+            return {k: enc(v) for k, v in x.items()}
+        if isinstance(x, (list, tuple)):
+            out = [enc(v) for v in x]
+            return {"__tuple__": out} if isinstance(x, tuple) else out
+        assert x is None or isinstance(x, (bool, int, float, str)), type(x)
+        return x
+
+    meta = json.dumps(enc(obj))
+    np.savez_compressed(os.path.join(GOLDEN, f"reference_{name}.npz"), meta=meta,
+                        data=np.frombuffer(b"".join(blob), np.uint8))
+
+
+def load_pin(name):
+    z = np.load(os.path.join(GOLDEN, f"reference_{name}.npz"), allow_pickle=False)
+    data = z["data"]
+
+    def dec(x):
+        if isinstance(x, dict):
+            if "__array__" in x:
+                dtype, shape, off = x["__array__"]
+                n = int(np.prod(shape)) * np.dtype(dtype).itemsize
+                return data[off:off + n].view(dtype).reshape(shape)
+            if "__tuple__" in x:
+                return tuple(dec(v) for v in x["__tuple__"])
+            return {k: dec(v) for k, v in x.items()}
+        if isinstance(x, list):
+            return [dec(v) for v in x]
+        return x
+
+    return dec(json.loads(str(z["meta"])))
+
+
+def digest(a, keep_dtype=True):
+    """A 64-bit sha256 prefix of an array's shape and bytes (and dtype; keep_dtype=False compares values only, as
+    float64): equal digests <=> np.array_equal (and the same dtype)."""
+    a = np.asarray(a.detach().cpu() if isinstance(a, torch.Tensor) else a)
+    if not keep_dtype:
+        a = a.astype(np.float64)
+    h = hashlib.sha256(f"{a.dtype.str if keep_dtype else ''}{a.shape}".encode())
+    h.update(np.ascontiguousarray(a).tobytes())
+    return h.hexdigest()[:16]
 
 
 def make_oracle(algo, cfg_dict, init_seed=0):

@@ -2,16 +2,12 @@
 value the caller passed: the mirrors are built with DISTINCT non-default values for every parameter the reference's
 signature has, and the struct `make_config(algo, **model._hyper(), **trainer._lrs)` produces is checked field by field.
 (The GPU parity fixtures mostly run the default values, where a parameter that never leaves Python would go
-unnoticed -- CPQ's KL weight did, once.)  Skipped where /root/reference is absent."""
-import inspect
-import sys
-
+unnoticed -- CPQ's KL weight did, once.)  The reference's signatures come from tests/golden/reference_surface.npz
+(tests/test_cpu_signatures.py: record_reference)."""
 import numpy as np
 import pytest
 
-from oracle import ref_shim
-
-pytestmark = pytest.mark.skipif(not ref_shim.available(), reason="reference tree not available")
+from tests import helpers
 
 O, A = 8, 2
 # reference parameter -> osrl_config field(s); None = not a step hyper-parameter of the engine (says why)
@@ -39,13 +35,8 @@ FIXED = {"time_emb": True, "use_rew": True, "use_cost": True, "cost_transform": 
 
 @pytest.fixture(scope="module")
 def ref_algos():
-    for m in [m for m in sys.modules if m == "osrl" or m.startswith("osrl.")]:
-        del sys.modules[m]
-    ref_shim.import_reference()
-    import osrl.algorithms as ra
-    yield ra
-    for m in [m for m in sys.modules if m == "osrl" or m.startswith("osrl.")]:
-        del sys.modules[m]
+    from tests.test_cpu_signatures import Recorded
+    return {k: [Recorded(*p) for p in v] for k, v in helpers.load_pin("surface").items()}
 
 
 def _distinct(name, default, salt):
@@ -82,14 +73,14 @@ def test_every_reference_hyperparameter_reaches_the_config(ref_algos, name):
     import osrl_b200.algorithms as mine
     from osrl_b200.engine import make_config
     kw, salt = {}, 0
-    for p in list(inspect.signature(getattr(ref_algos, name).__init__).parameters.values())[1:]:
+    for p in ref_algos[name]:
         if p.name == "device":
             continue
         salt += 1
         kw[p.name] = _distinct(p.name, p.default, salt)
     model = getattr(mine, name)(device="cpu", **kw)
     tkw = {}
-    for p in list(inspect.signature(getattr(ref_algos, name + "Trainer").__init__).parameters.values())[1:]:
+    for p in ref_algos[name + "Trainer"]:
         if p.name in NOT_CONFIG and p.name not in FIXED:
             continue
         salt += 1

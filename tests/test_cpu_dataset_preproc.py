@@ -2,32 +2,26 @@
 reference (osrl/common/dataset.py) on seeded synthetic data: process_bc_dataset (all modes incl. the Pareto frontier),
 SequenceDataset with the reference's default Pareto-frontier augmentation, random augmentation, pf_only and the
 sampling-probability variants.  The reference needs `oapackage` for the frontier; tests/stubs/oapackage.py restates
-its two classes (brute-force non-dominated set).  Skipped where /root/reference is absent."""
-import os
+its two classes (brute-force non-dominated set).  What the reference computes is stored in
+tests/golden/reference_dataset.npz (record_reference below, run by oracle/record_reference.py): arrays compared for
+equality as sha256 digests; of SequenceDataset's relabelled targets and start probabilities, every trajectory's first
+target and the whole of a fixed sample of trajectories; everything else as is."""
 import random
-import sys
 
 import numpy as np
 import pytest
 
-from oracle import ref_shim, synth
+from oracle import synth
+from tests import helpers
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-pytestmark = pytest.mark.skipif(not ref_shim.available(), reason="reference tree not available")
+MODES = ["all", "multi-task", "safe", "risky", "boundary", "frontier"]
+GAMMAS = [1.0, 0.99]
+TRAJ_SAMPLE = 64       # trajectories of each SequenceDataset case stored whole
 
 
 @pytest.fixture(scope="module")
 def ref_dataset():
-    sys.path.insert(0, os.path.join(ROOT, "tests", "stubs"))
-    import oapackage  # noqa: F401  (the stub; must be importable before the reference module is)
-    for m in [m for m in sys.modules if m == "osrl" or m.startswith("osrl.")]:
-        del sys.modules[m]
-    osrl = ref_shim.import_reference()
-    import osrl.common.dataset as rd
-    if not hasattr(rd, "oapackage"):
-        rd.oapackage = oapackage
-    yield rd
-    sys.path.remove(os.path.join(ROOT, "tests", "stubs"))
+    return helpers.load_pin("dataset")
 
 
 def _data(seed=3, eps=60, T=37):
@@ -49,17 +43,21 @@ def test_pareto_front_matches_brute_force():
         assert brute == pareto_front_2d(c, r)
 
 
-@pytest.mark.parametrize("mode", ["all", "multi-task", "safe", "risky", "boundary", "frontier"])
-@pytest.mark.parametrize("gamma", [1.0, 0.99])
+def bc_columns(process_bc_dataset, mode, gamma):
+    b = {k: v.copy() for k, v in _data().items()}
+    process_bc_dataset(b, 6, gamma, mode)
+    return {k: (v.dtype.str, helpers.digest(v, keep_dtype=False)) for k, v in b.items()}
+
+
+@pytest.mark.parametrize("mode", MODES)
+@pytest.mark.parametrize("gamma", GAMMAS)
 def test_process_bc_dataset(ref_dataset, mode, gamma):
     from osrl_b200.common.dataset import process_bc_dataset
-    d = _data()
-    a, b = {k: v.copy() for k, v in d.items()}, {k: v.copy() for k, v in d.items()}
-    ref_dataset.process_bc_dataset(a, 6, gamma, mode)
-    process_bc_dataset(b, 6, gamma, mode)
+    a = ref_dataset["bc"][f"{mode}/{gamma}"]
+    b = bc_columns(process_bc_dataset, mode, gamma)
     assert set(a) == set(b)
     for k in a:
-        assert a[k].dtype == b[k].dtype and np.array_equal(a[k], b[k]), (mode, gamma, k)
+        assert tuple(a[k]) == b[k], (mode, gamma, k)
 
 
 CASES = {
@@ -74,38 +72,85 @@ CASES = {
 }
 
 
+def _sequence_dataset(cls, case):
+    d = _data(seed=5, eps=900, T=16)   # enough trajectories for the 10 x 50 outlier grid (bins of <= 2 are dropped)
+    np.random.seed(7); random.seed(7)
+    return cls({k: v.copy() for k, v in d.items()}, seq_len=10, reward_scale=0.1, cost_scale=1.0, **CASES[case])
+
+
+def _windows(ds):
+    np.random.seed(11); random.seed(11)
+    return [x for _, x in zip(range(5), iter(ds))]
+
+
+def _sources_digest(trajs):
+    """one digest of every trajectory's (observations, actions, costs), compared by value"""
+    return helpers.digest(np.array([helpers.digest(x, keep_dtype=False) for t in trajs for x in t]))
+
+
+def record_sequence_case(SequenceDataset, case):
+    ref = _sequence_dataset(SequenceDataset, case)
+    trajs = ref.dataset
+    first = np.array([[t["returns"][0], t["cost_returns"][0]] for t in trajs])
+    sample = np.sort(np.random.default_rng(0).choice(len(trajs), min(TRAJ_SAMPLE, len(trajs)), replace=False))
+    out = {"n": len(trajs), "lengths": np.array([len(t["returns"]) for t in trajs], np.int64),
+           "sources": _sources_digest([(t["observations"], t["actions"], t["costs"]) for t in trajs]),
+           "first": first, "sample": sample,
+           "sample_returns": [np.asarray(trajs[i]["returns"]) for i in sample],
+           "sample_cost_returns": [np.asarray(trajs[i]["cost_returns"]) for i in sample],
+           "sample_prob": None if ref.sample_prob is None else np.asarray(ref.sample_prob),
+           "windows": [tuple(np.asarray(u) for u in x) for x in _windows(ref)]}
+    if CASES[case].get("start_sampling"):
+        out["n_start_idx_sample_prob"] = len(ref.start_idx_sample_prob)
+        out["start_idx_sample_prob"] = [np.asarray(ref.start_idx_sample_prob[i]) for i in sample]
+    return out
+
+
 @pytest.mark.parametrize("case", sorted(CASES))
 def test_sequence_dataset_modes(ref_dataset, case):
     """Same seeds -> same trajectories (sources, relabelled return / cost to go), same sampling probabilities, and the
     same windows from the iterator."""
     from osrl_b200.common.dataset import SequenceDataset
-    kw = CASES[case]
-    d = _data(seed=5, eps=900, T=16)   # enough trajectories for the 10 x 50 outlier grid (bins of <= 2 are dropped)
-    np.random.seed(7); random.seed(7)
-    ref = ref_dataset.SequenceDataset({k: v.copy() for k, v in d.items()}, seq_len=10, reward_scale=0.1, cost_scale=1.0, **kw)
-    np.random.seed(7); random.seed(7)
-    mine = SequenceDataset({k: v.copy() for k, v in d.items()}, seq_len=10, reward_scale=0.1, cost_scale=1.0, **kw)
-    assert len(ref.dataset) == len(mine)
-    for i, t in enumerate(ref.dataset):
-        lo, hi, rtg, ctg = mine._traj[i]
-        assert np.array_equal(t["observations"], mine._obs[lo:hi]) and np.array_equal(t["actions"], mine._act[lo:hi]), (case, i)
-        assert np.array_equal(t["costs"], mine._cost[lo:hi]), (case, i)
-        # (relabelled targets: the frontier fit sees the same points in a different order -- 1e-6 relative)
-        assert np.allclose(t["returns"], rtg, rtol=2e-6, atol=1e-5) and np.allclose(t["cost_returns"], ctg, rtol=2e-6, atol=1e-5), (case, i)
-    if ref.sample_prob is None:
+    ref = ref_dataset["seq"][case]
+    mine = _sequence_dataset(SequenceDataset, case)
+    assert ref["n"] == len(mine)
+    assert np.array_equal(ref["lengths"], [hi - lo for lo, hi, _, _ in mine._traj]), case
+    assert ref["sources"] == _sources_digest([(mine._obs[lo:hi], mine._act[lo:hi], mine._cost[lo:hi])
+                                              for lo, hi, _, _ in mine._traj]), case
+    # (relabelled targets: the frontier fit sees the same points in a different order -- 1e-6 relative)
+    rtol, atol = 2e-6, 1e-5
+    rtg = [np.asarray(t[2]) for t in mine._traj]
+    ctg = [np.asarray(t[3]) for t in mine._traj]
+    got_first = np.array([[r[0], c[0]] for r, c in zip(rtg, ctg)])
+    assert np.allclose(ref["first"], got_first, rtol=rtol, atol=atol), case
+    for i, w_r, w_c in zip(ref["sample"], ref["sample_returns"], ref["sample_cost_returns"]):
+        assert np.allclose(w_r, rtg[i], rtol=rtol, atol=atol) and np.allclose(w_c, ctg[i], rtol=rtol, atol=atol), (case, i)
+    if ref["sample_prob"] is None:
         assert mine.sample_prob is None
     else:
-        assert np.allclose(ref.sample_prob, mine.sample_prob, rtol=1e-5, atol=1e-9)
-    if kw.get("start_sampling"):
-        for a, b in zip(ref.start_idx_sample_prob, mine.start_idx_sample_prob):
-            assert np.allclose(a, b, rtol=1e-6)
-    np.random.seed(11); random.seed(11)
-    ra = [x for _, x in zip(range(5), iter(ref))]
-    np.random.seed(11); random.seed(11)
-    ma = [x for _, x in zip(range(5), iter(mine))]
-    for x, y in zip(ra, ma):
+        assert np.allclose(ref["sample_prob"], mine.sample_prob, rtol=1e-5, atol=1e-9)
+    if CASES[case].get("start_sampling"):
+        assert ref["n_start_idx_sample_prob"] == len(mine.start_idx_sample_prob)
+        for i, a in zip(ref["sample"], ref["start_idx_sample_prob"]):
+            assert np.allclose(a, mine.start_idx_sample_prob[i], rtol=1e-6)
+    for x, y in zip(ref["windows"], _windows(mine), strict=True):
         for u, v in zip(x, y):
             assert np.asarray(u).dtype == np.asarray(v).dtype and np.allclose(u, v, rtol=2e-6, atol=1e-5), case
+
+
+SPLIT_KEYS = ("observations", "actions", "rewards", "costs", "returns", "cost_returns")
+
+
+def _split_data():
+    d = _data(seed=9, eps=40, T=23)
+    rng = np.random.default_rng(2)
+    d["costs"] = np.where(rng.random(d["costs"].shape) < 0.5, d["costs"], rng.random(d["costs"].shape)).astype(np.float32)
+    d["terminals"][40] = True
+    return d
+
+
+def _split_digests(trajs):
+    return [[(t[k].dtype.str, helpers.digest(t[k], keep_dtype=False)) for k in SPLIT_KEYS] for t in trajs]
 
 
 @pytest.mark.parametrize("cost_reverse", [False, True])
@@ -114,16 +159,28 @@ def test_oracle_split_trajectories_is_the_reference(ref_dataset, cost_reverse):
     against the unmodified process_sequence_dataset (dataset.py:137-183), bit for bit, with fractional costs, a
     trailing unfinished episode and both end flags."""
     from oracle import cdt as ocdt
-    d = _data(seed=9, eps=40, T=23)
-    rng = np.random.default_rng(2)
-    d["costs"] = np.where(rng.random(d["costs"].shape) < 0.5, d["costs"], rng.random(d["costs"].shape)).astype(np.float32)
-    d["terminals"][40] = True
-    want, _ = ref_dataset.process_sequence_dataset({k: v.copy() for k, v in d.items()}, cost_reverse)
-    got = ocdt.split_trajectories(d, cost_reverse)
+    want = ref_dataset["split"][str(cost_reverse)]
+    got = _split_digests(ocdt.split_trajectories(_split_data(), cost_reverse))
     assert len(want) == len(got)
     for w, g in zip(want, got):
-        for k in ("observations", "actions", "rewards", "costs", "returns", "cost_returns"):
-            assert w[k].dtype == g[k].dtype and np.array_equal(w[k], g[k]), k
+        for k, wk, gk in zip(SPLIT_KEYS, w, g):
+            assert tuple(wk) == gk, k
+
+
+def _transition_data():
+    d = _data(seed=4, eps=12, T=9)
+    d["terminals"][20] = True
+    return d
+
+
+def _transition_record(ds, state_init):
+    np.random.seed(2)
+    it = iter(ds)
+    out = {"columns": {k: ds.dataset[k] for k in ("done",) + (("is_init",) if state_init else ())},
+           "stream": [tuple(np.asarray(x) for x in next(it)) for _ in range(25)]}
+    if state_init:
+        out["states"] = [np.asarray(x) for x in ds.get_dataset_states()]
+    return out
 
 
 @pytest.mark.parametrize("state_init", [False, True])
@@ -131,22 +188,23 @@ def test_transition_dataset_stream_is_the_reference(ref_dataset, state_init):
     """TransitionDataset (dataset.py:790-847): done / is_init columns, the float32 scaling of rewards and costs, the
     tuple layout and the index stream of __iter__ under the same numpy seed; get_dataset_states for COptiDICE."""
     from osrl_b200.common.dataset import TransitionDataset
-    d = _data(seed=4, eps=12, T=9)
-    d["terminals"][20] = True
-    a = ref_dataset.TransitionDataset({k: v.copy() for k, v in d.items()}, 0.1, 3.0, state_init)
-    b = TransitionDataset({k: v.copy() for k, v in d.items()}, 0.1, 3.0, state_init)
-    for k in ("done",) + (("is_init",) if state_init else ()):
-        assert a.dataset[k].dtype == b.dataset[k].dtype and np.array_equal(a.dataset[k], b.dataset[k]), k
-    np.random.seed(2)
-    ia = iter(a)
-    want = [next(ia) for _ in range(25)]
-    np.random.seed(2)
-    ib = iter(b)
-    got = [next(ib) for _ in range(25)]
-    for w, g in zip(want, got):
+    a = ref_dataset["transition"][str(state_init)]
+    b = _transition_record(TransitionDataset(_transition_data(), 0.1, 3.0, state_init), state_init)
+    for k, w in a["columns"].items():
+        assert w.dtype == b["columns"][k].dtype and np.array_equal(w, b["columns"][k]), k
+    for w, g in zip(a["stream"], b["stream"], strict=True):
         assert len(w) == len(g) == (7 if state_init else 6)
         for x, y in zip(w, g):
-            assert np.asarray(x).dtype == np.asarray(y).dtype and np.array_equal(x, y)
+            assert x.dtype == y.dtype and np.array_equal(x, y)
     if state_init:
-        for x, y in zip(a.get_dataset_states(), b.get_dataset_states()):
-            assert np.array_equal(np.asarray(x), np.asarray(y))
+        for x, y in zip(a["states"], b["states"], strict=True):
+            assert np.array_equal(x, y)
+
+
+def record_reference(osrl):
+    rd = osrl.common.dataset
+    return {"bc": {f"{m}/{g}": bc_columns(rd.process_bc_dataset, m, g) for m in MODES for g in GAMMAS},
+            "seq": {case: record_sequence_case(rd.SequenceDataset, case) for case in sorted(CASES)},
+            "split": {str(c): _split_digests(rd.process_sequence_dataset(_split_data(), c)[0]) for c in (False, True)},
+            "transition": {str(s): _transition_record(rd.TransitionDataset(_transition_data(), 0.1, 3.0, s), s)
+                           for s in (False, True)}}

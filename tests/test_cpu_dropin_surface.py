@@ -2,9 +2,9 @@
 alias package (compat/osrl), and every keyword they pass to those classes / functions is accepted by the mirrors.
 
 The scripts are parsed, not executed (they need a GPU for our models): for each `examples/train/*.py` and
-`examples/eval/*.py` of the reference the test collects `from osrl... import X` and the calls `X(...)` /
-`trainer.method(...)`, and checks them against `inspect.signature` of the mirror.  Skipped where /root/reference is
-absent (the GPU box); the executable counterpart is tests/test_gpu_dropin_loop.py."""
+`examples/eval/*.py` of the reference, record_reference collects `from osrl... import X` and the calls `X(...)` /
+`trainer.method(...)` / `model.method(...)` into tests/golden/reference_scripts.npz, and the test checks them against
+`inspect.signature` of the mirror; the executable counterpart is tests/test_gpu_dropin_loop.py."""
 import ast
 import glob
 import inspect
@@ -13,11 +13,37 @@ import sys
 
 import pytest
 
+from tests import helpers
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.environ.get("OSRL_REFERENCE_ROOT", "/root/reference")
-SCRIPTS = sorted(glob.glob(os.path.join(REF, "examples", "train", "train_*.py")) +
-                 glob.glob(os.path.join(REF, "examples", "eval", "eval_*.py")))
-pytestmark = pytest.mark.skipif(not SCRIPTS, reason="reference tree not available")
+SCRIPTS = [f"{kind}_{algo}.py" for kind in ("eval", "train") for algo in ("bc", "bcql", "bearl", "cdt", "coptidice", "cpq")]
+
+
+def record_reference(osrl):
+    """{script: {"imports": [(module, name, asname)], "calls": [(receiver or None, function, keywords, n_positional)]}}"""
+    from oracle import ref_shim
+    ref = ref_shim.REFERENCE_ROOT
+    out = {}
+    for path in sorted(glob.glob(os.path.join(ref, "examples", "train", "train_*.py")) +
+                       glob.glob(os.path.join(ref, "examples", "eval", "eval_*.py"))):
+        tree = ast.parse(open(path).read())
+        imports, calls = [], []
+        for node in ast.walk(tree):
+            if isinstance(node, ast.ImportFrom) and node.module and node.module.startswith("osrl"):
+                imports += [(node.module, a.name, a.asname) for a in node.names]
+        names = {asname or name for _, name, asname in imports}
+        for node in ast.walk(tree):
+            if not isinstance(node, ast.Call):
+                continue
+            kwargs = [k.arg for k in node.keywords if k.arg]
+            if isinstance(node.func, ast.Name) and node.func.id in names:
+                calls.append((None, node.func.id, kwargs, len(node.args)))
+            elif isinstance(node.func, ast.Attribute) and isinstance(node.func.value, ast.Name) and \
+                    node.func.value.id in ("trainer", "model"):
+                calls.append((node.func.value.id, node.func.attr, kwargs, len(node.args)))
+        out[os.path.basename(path)] = {"imports": imports, "calls": calls}
+    assert sorted(out) == SCRIPTS, sorted(out)
+    return out
 
 
 @pytest.fixture(scope="module")
@@ -50,37 +76,33 @@ def _accepts(fn, kwargs, n_pos):
     return names_ok and (n_pos <= len(positional) or any(p.kind == p.VAR_POSITIONAL for p in params.values()))
 
 
-@pytest.mark.parametrize("script", SCRIPTS, ids=[os.path.basename(s) for s in SCRIPTS])
-def test_script_surface(alias, script):
+@pytest.fixture(scope="module")
+def scripts():
+    return helpers.load_pin("scripts")
+
+
+@pytest.mark.parametrize("script", SCRIPTS)
+def test_script_surface(alias, scripts, script):
     import importlib
-    tree = ast.parse(open(script).read())
+    rec = scripts[script]
     imported = {}
-    for node in ast.walk(tree):
-        if isinstance(node, ast.ImportFrom) and node.module and node.module.startswith("osrl"):
-            mod = importlib.import_module(node.module)
-            for a in node.names:
-                assert hasattr(mod, a.name), f"{os.path.basename(script)}: {node.module}.{a.name} missing"
-                imported[a.asname or a.name] = getattr(mod, a.name)
+    for module, name, asname in rec["imports"]:
+        mod = importlib.import_module(module)
+        assert hasattr(mod, name), f"{script}: {module}.{name} missing"
+        imported[asname or name] = getattr(mod, name)
     assert imported, "script imports nothing from osrl?"
     trainer_cls = [v for k, v in imported.items() if k.endswith("Trainer")]
     checked = 0
-    for node in ast.walk(tree):
-        if not isinstance(node, ast.Call):
-            continue
-        kwargs = [k.arg for k in node.keywords if k.arg]
-        if isinstance(node.func, ast.Name) and node.func.id in imported:
-            target = imported[node.func.id]
+    for receiver, func, kwargs, n_args in rec["calls"]:
+        if receiver is None and func in imported:
+            target = imported[func]
             fn = target.__init__ if inspect.isclass(target) else target
-            assert _accepts(fn, kwargs, len(node.args)), \
-                f"{os.path.basename(script)}: {node.func.id}({', '.join(kwargs)}) not accepted by {fn}"
+            assert _accepts(fn, kwargs, n_args), f"{script}: {func}({', '.join(kwargs)}) not accepted by {fn}"
             checked += 1
-        elif isinstance(node.func, ast.Attribute) and isinstance(node.func.value, ast.Name) and \
-                node.func.value.id == "trainer" and trainer_cls:
-            assert hasattr(trainer_cls[0], node.func.attr), f"{os.path.basename(script)}: trainer.{node.func.attr} missing"
-            assert _accepts(getattr(trainer_cls[0], node.func.attr), kwargs, len(node.args)), \
-                f"{os.path.basename(script)}: trainer.{node.func.attr} call not accepted"
+        elif receiver == "trainer" and trainer_cls:
+            assert hasattr(trainer_cls[0], func), f"{script}: trainer.{func} missing"
+            assert _accepts(getattr(trainer_cls[0], func), kwargs, n_args), f"{script}: trainer.{func} call not accepted"
             checked += 1
-        elif isinstance(node.func, ast.Attribute) and isinstance(node.func.value, ast.Name) and \
-                node.func.value.id == "model" and node.func.attr in ("load_state_dict", "state_dict", "to", "eval", "parameters"):
+        elif receiver == "model" and func in ("load_state_dict", "state_dict", "to", "eval", "parameters"):
             checked += 1   # nn.Module API: the mirrors are nn.Modules
-    assert checked >= 3, f"{os.path.basename(script)}: only {checked} calls recognised"
+    assert checked >= 3, f"{script}: only {checked} calls recognised"

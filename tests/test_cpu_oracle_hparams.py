@@ -3,14 +3,13 @@
 moved off its default -- discount, Polyak rate, perturbation range, the two lambdas, KL weight, ensemble sizes 1 and 3,
 sample counts, episode length, cost limits on both sides of the batch's Qc, PID gains, CPQ's threshold scalar, BEAR's
 Laplacian kernel / sigma / MMD threshold / delayed policy start -- so that a GPU parity run at such a configuration
-compares against something that was itself compared.  Skipped where /root/reference is absent."""
-import sys
-
+compares against something that was itself compared.  The reference's runs are stored in
+tests/golden/reference_hparams.npz (record_reference below, run by oracle/record_reference.py: stats in full, initial
+parameters as digests, each final tensor as its max |x|, checksum and a fixed sample of entries)."""
 import pytest
 
-from oracle import algos, ref_shim
-
-pytestmark = pytest.mark.skipif(not ref_shim.available(), reason="reference tree not available")
+from oracle import algos, make_golden
+from tests import helpers
 
 TWISTED = {
     "bc_t": ("bc", algos.BCConfig(9, 3, 2.0, [24, 40], 3e-3), 12, 3),
@@ -41,20 +40,13 @@ TWISTED = {
 
 @pytest.fixture(scope="module")
 def osrl_ref():
-    for m in [m for m in sys.modules if m == "osrl" or m.startswith("osrl.")]:
-        del sys.modules[m]
-    osrl = ref_shim.import_reference()
-    yield osrl
-    for m in [m for m in sys.modules if m == "osrl" or m.startswith("osrl.")]:
-        del sys.modules[m]
+    return helpers.load_pin("hparams")
 
 
 @pytest.mark.parametrize("name", list(TWISTED))
-def test_oracle_equals_reference_off_the_defaults(osrl_ref, name, tmp_path, monkeypatch):
-    from oracle import make_golden
+def test_oracle_equals_reference_off_the_defaults(osrl_ref, name):
     algo, cfg, B, steps = TWISTED[name]
-    monkeypatch.setattr(make_golden, "OUT", str(tmp_path))     # the comparison is the point; the fixture is thrown away
-    make_golden.run_case(osrl_ref, name, algo, cfg, B, steps, True)
+    make_golden.check_run(name, osrl_ref[name], make_golden.oracle_run(algo, cfg, B, steps), 2e-6, 1e-12, 2e-6)
 
 
 CDT_TWISTED = {
@@ -69,15 +61,17 @@ CDT_TWISTED = {
 
 
 @pytest.mark.parametrize("name", list(CDT_TWISTED))
-def test_cdt_oracle_equals_reference_off_the_defaults(osrl_ref, name, tmp_path, monkeypatch):
-    """oracle/cdt.py against the unmodified CDT / CDTTrainer (run_cdt_case asserts stats and parameters): other window
+def test_cdt_oracle_equals_reference_off_the_defaults(osrl_ref, name):
+    """oracle/cdt.py against the unmodified CDT / CDTTrainer (check_cdt_run asserts stats and parameters): other window
     length, width, head count, temperature, AdamW betas / decay, clip threshold on both sides of the gradient norm,
     warm-up, both auxiliary loss weights, and replayed dropout at three different rates."""
-    from oracle import cdt as ocdt
-    from oracle import make_golden
     kw, B, steps = CDT_TWISTED[name]
-    monkeypatch.setattr(make_golden, "OUT", str(tmp_path))
-    make_golden.run_cdt_case(osrl_ref, name, ocdt.CDTConfig(**kw), B, steps, True)
+    make_golden.check_cdt_run(name, osrl_ref[name], make_golden.oracle_cdt_run(_cdt(**kw), B, steps))
+
+
+def _cdt(**kw):
+    from oracle import cdt as ocdt
+    return ocdt.CDTConfig(**kw)
 
 
 def _cop(**kw):
@@ -99,11 +93,26 @@ COP_TWISTED = {
 
 
 @pytest.mark.parametrize("name", list(COP_TWISTED))
-def test_coptidice_oracle_equals_reference_off_the_defaults(osrl_ref, name, tmp_path, monkeypatch):
-    """oracle/coptidice.py against the unmodified COptiDICE.update (run_coptidice_case asserts stats, parameters, tau
+def test_coptidice_oracle_equals_reference_off_the_defaults(osrl_ref, name):
+    """oracle/coptidice.py against the unmodified COptiDICE.update (check_coptidice_run asserts stats, parameters, tau
     and lambda): all three f-divergences (the committed fixture is softchi only), ensemble sizes 1..3, discount, alpha,
     the cost upper-bound epsilon incl. 0, initial-state proportion, cost limits and the three learning rates."""
-    from oracle import make_golden
     kw, B, steps = COP_TWISTED[name]
-    monkeypatch.setattr(make_golden, "OUT", str(tmp_path))
-    make_golden.run_coptidice_case(osrl_ref, name, _cop(**kw), B, steps)
+    make_golden.check_coptidice_run(name, osrl_ref[name], make_golden.oracle_coptidice_run(_cop(**kw), B, steps))
+
+
+def record_reference(osrl):
+    out = {}
+    for name, (algo, cfg, B, steps) in TWISTED.items():
+        run = make_golden.reference_run(osrl, algo, cfg, B, steps)
+        make_golden.check_run(name, run, make_golden.oracle_run(algo, cfg, B, steps), 2e-6, 1e-12, 2e-6)
+        out[name] = make_golden.pin_run(run)
+    for name, (kw, B, steps) in CDT_TWISTED.items():
+        run = make_golden.reference_cdt_run(osrl, _cdt(**kw), B, steps)
+        make_golden.check_cdt_run(name, run, make_golden.oracle_cdt_run(_cdt(**kw), B, steps))
+        out[name] = make_golden.pin_run(run)
+    for name, (kw, B, steps) in COP_TWISTED.items():
+        run = make_golden.reference_coptidice_run(osrl, _cop(**kw), B, steps)
+        make_golden.check_coptidice_run(name, run, make_golden.oracle_coptidice_run(_cop(**kw), B, steps))
+        out[name] = make_golden.pin_run(run)
+    return out
